@@ -9,6 +9,9 @@ One "step" = one decoded token = one pass of the hot path (225 quantized matvecs
   roofline : the dominant kernel (the ffn_gate/ffn_up-shaped matvec, 11008x4096) timed with CUDA events
   cpu_baseline : the CPU restatement of the reference's AVX2 path (oracle/, all host threads) on a bounded sample
 `--impl reference` runs ONLY that CPU path and prints the same line shape.
+`--dump-outputs DIR` writes what the timed path computed in its last timed step (logits as float32, token ids as float64, a
+fixed seeded sample of the prefill GEMM outputs) to DIR/<name>.npy; the inputs are seeded, so two builds run with the same
+arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -207,9 +210,17 @@ def run_reference(args, rank, world):
     print(json.dumps(line))
 
 
-def quick_decode(workload: str, local_rank: int, K: int, W: int, start_pos: int):
+def write_outputs(directory: str, arrays: dict):
+    os.makedirs(directory, exist_ok=True)
+    for name, a in arrays.items():
+        a = np.asarray(a)
+        np.save(os.path.join(directory, f"{name}.npy"), a.astype(np.float64 if a.dtype.kind in "iu" else np.float32))
+
+
+def quick_decode(workload: str, local_rank: int, K: int, W: int, start_pos: int, outputs: dict | None = None):
     """Second measurement of the default run: the same decode loop (device-resident and e2e) for another weight type, so that one
-    bench line covers the whole metric (Q8_0 AND Q4_0).  Returns a dict that is embedded in the main JSON line."""
+    bench line covers the whole metric (Q8_0 AND Q4_0).  Returns a dict that is embedded in the main JSON line; `outputs`, when
+    given, receives the logits of the last timed e2e step."""
     from crabml_b200 import CudaTensorDevice
     from crabml_b200 import runner as R
     cname, wt_name, ct_name = WORKLOADS[workload]
@@ -235,6 +246,8 @@ def quick_decode(workload: str, local_rank: int, K: int, W: int, start_pos: int)
         for _ in range(K):
             tok = step_e2e(tok, pos); pos += 1
         e2e_ms = max(dev.timer_end(), (time.perf_counter() - t0) * 1e3)
+        if outputs is not None:
+            outputs[f"{workload}_logits"] = runner.logits.copy()
         pos = p0
         l0 = dev.launch_count()
         dev.timer_begin()
@@ -339,6 +352,8 @@ def run_b200(args, rank, world, local_rank):
     for _ in range(K):
         tok = step_e2e(tok, pos); pos += 1
     e2e_sync_ms = max_over_ranks(max(dev.timer_end(), (time.perf_counter() - t0) * 1e3))
+    # what the callers of the two e2e regions received in the last step (the device-resident region exports nothing)
+    outputs = {"logits": lgs[-1], "token_ids": ids, "logits_synchronous": runner.logits.copy()}
     pos = p0
     barrier()
     # ---- timed region 2: device-resident (no per-step host<->device traffic) -----------------------------------
@@ -355,6 +370,9 @@ def run_b200(args, rank, world, local_rank):
     launches_val = dev.launch_count() - launches1
     clocks = sampler.stop()
     barrier()
+    # the runner keeps no copy of the logits of an export=False step: repeat the region's last step (same token, same position,
+    # same call) with the export, untimed
+    outputs["logits_device_resident"] = runner.forward([toks[-1]], pos - 1, export=True).copy()
 
     # ---- roofline of the dominant kernel: ffn_gate/ffn_up-shaped matvec over all layers' weights (>> L2) ----------
     # (timed through an eager-mode device handle on the same GPU so that each matmul_vec is its own launch pair)
@@ -436,9 +454,11 @@ def run_b200(args, rank, world, local_rank):
             # run `--workload llama2-7b-q4_0-q6k` for that variant)
             weights = None
             try:
-                line["also"] = {"llama2-7b-q4_0": quick_decode("llama2-7b-q4_0", local_rank, K, W, args.start_pos)}
+                line["also"] = {"llama2-7b-q4_0": quick_decode("llama2-7b-q4_0", local_rank, K, W, args.start_pos, outputs)}
             except Exception as e:      # the second block must never cost the main line
                 line["also"] = {"llama2-7b-q4_0": {"error": repr(e)}}
+        if args.dump_outputs:
+            write_outputs(args.dump_outputs, outputs)
         print(json.dumps(line))
     if dist is not None:
         dist.destroy_process_group()
@@ -473,11 +493,11 @@ def run_prefill(args, rank, world, local_rank):
     wbytes = sum(R.weight_bytes(t.dtype(), *t.shape()) for key in ("wq", "wk", "wv", "wo", "ffn_gate", "ffn_up", "ffn_down") for t in weights[key])
 
     def step():
+        """-> classifier output and the outputs of the last layer's seven GEMMs (the other layers' are dropped at once)."""
         for l in range(conf.n_layers):
-            for key in ("wq", "wk", "wv", "wo", "ffn_gate", "ffn_up"):
-                weights[key][l].matmul_vec(x_dim)
-            weights["ffn_down"][l].matmul_vec(x_hid)
-        return weights["output_weight"].matmul_vec(x_last)
+            last = {key: weights[key][l].matmul_vec(x_dim) for key in ("wq", "wk", "wv", "wo", "ffn_gate", "ffn_up")}
+            last["ffn_down"] = weights["ffn_down"][l].matmul_vec(x_hid)
+        return weights["output_weight"].matmul_vec(x_last), last
     K, W = args.steps, args.warmup
     for _ in range(W):
         step()
@@ -486,7 +506,7 @@ def run_prefill(args, rank, world, local_rank):
     l0 = dev.launch_count()
     dev.timer_begin()
     for _ in range(K):
-        step()
+        logits, gemms = step()
     ms = dev.timer_end()
     launches = dev.launch_count() - l0
     # e2e: what crosses the host boundary in a prompt pass -- the token ids go host->device (the embedding rows are gathered on the
@@ -522,6 +542,11 @@ def run_prefill(args, rank, world, local_rank):
                          "achieved": tf, "peak": peak_tf, "peak_source": peak_src + " bf16_tflops_sustained", "unit": "TFLOP/s", "frac": tf / peak_tf, "traffic": None,
                          "note": "whole step (dequantise + quantise + GEMM launches) over the dense FLOPs; the GEMM kernel alone is profiled in profiles/"},
             "clocks": clocks}
+    if args.dump_outputs:
+        pick = np.random.default_rng(SEED)          # the same 4096 elements of each [b, rows] product in every run
+        write_outputs(args.dump_outputs, {"logits": logits.export(),
+                                          **{f"{key}_sample": y.export()[np.sort(pick.choice(b * y.shape()[1], 4096, replace=False))]
+                                             for key, y in gemms.items()}})
     print(json.dumps(line))
     dev.close()
 
@@ -540,7 +565,12 @@ def main():
     ap.add_argument("--no-also", action="store_true", help="skip the second (Q4_0) measurement of the default run")
     ap.add_argument("--multi", default="sharded", choices=["sharded", "replicas"], help="N > 1: shard one token stream (strong scaling, default) or run N independent replicas")
     ap.add_argument("--comm", default="p2p", choices=["p2p", "nccl"], help="exchange transport of the sharded path: one-shot NVLink peer stores (default) or the NCCL baseline")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs needs --impl b200")
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))

@@ -13,20 +13,11 @@ def pytest_configure(config):
 
 
 def find_fixture(name):
-    """GGUF fixtures are the reference's testdata; they are copied (git-ignored) into
-    oracle/_ref/testdata by __graft_entry__.build() so that they travel to the GPU box."""
-    for d in (os.path.join(ROOT, "oracle", "_ref", "testdata"), "/root/reference/testdata"):
-        p = os.path.join(d, name)
-        if os.path.exists(p):
-            return p
-    return None
+    """Path of a GGUF test model: the synthetic stand-ins for tinyllamas-stories-15M of tests/synth_model.py."""
+    from tests.synth_model import model_path
+    return model_path(name)
 
 
 @pytest.fixture
 def fixture_path():
-    def _get(name):
-        p = find_fixture(name)
-        if p is None:
-            pytest.skip(f"fixture {name} not available (run __graft_entry__.build() where /root/reference exists)")
-        return p
-    return _get
+    return find_fixture

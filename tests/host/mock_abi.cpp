@@ -1,8 +1,8 @@
 // Mock of the C ABI (include/crabml_cuda.h) for the host-logic test of the C++ Llama2Runner replay
 // (crabml_b200/csrc/host/llama2_runner.cpp): every entry point the runner uses only RECORDS the call (op name + views) into
 // a trace; no CUDA, no arithmetic.  tests/test_host_runner_trace.py builds llama2_runner.cpp against this file and compares
-// the trace with the one the Python replay of the reference's forward() (oracle/llama_replay.py, which reproduces the
-// reference's golden generations on the CPU oracle) produces on a trace-only tensor class.
+// the trace with the one the Python replay of the reference's forward() (oracle/llama_replay.py, which reproduced the
+// reference's golden generations on its trained models) produces on a trace-only tensor class.
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>

@@ -1,6 +1,6 @@
-"""End-to-end parity on the reference's own GGUF fixtures: the Llama2Runner replay
+"""End-to-end parity on the GGUF test models (stand-ins for the reference's fixtures, tests/synth_model.py): the Llama2Runner replay
 (llama2.rs:184-281,527-638) over CudaTensor vs the same replay over the CPU oracle.
-north_star: logits within 1e-3 relative; golden generations of llama2.rs:673-703 reproduced."""
+north_star: logits within 1e-3 relative; the test models' golden generations (tests/test_oracle_golden_text.py) reproduced."""
 import numpy as np
 import pytest
 
@@ -50,7 +50,7 @@ def test_exact_order_mode_is_bit_identical(fixture_path, fname, text, ids, f16_k
         g_out, g_logits = _run(CudaTensor, gdev, gm, 11, f16_kv)
         o_out, o_logits = _run(OracleTensor, odev, gm, 11, f16_kv)
         assert g_out == o_out
-        if not f16_kv or "q8_0" in fname:                     # llama2.rs:673-719 golden strings
+        if not f16_kv or "q8_0" in fname:                     # golden generation
             assert g_out == ids and decode_text(tok, g_out) == text
         rel = (np.abs(g_logits - o_logits) / np.abs(o_logits).max(axis=1, keepdims=True)).max()
         assert rel < REL_TOL, rel
@@ -66,7 +66,7 @@ def test_exact_order_mode_is_bit_identical(fixture_path, fname, text, ids, f16_k
 
 @pytest.mark.parametrize("fname,text,ids", CASES)
 def test_fast_mode_generation_and_band(fixture_path, fname, text, ids):
-    """Fast (warp-parallel) kernels: same greedy text as the reference's golden strings, and logits no
+    """Fast (warp-parallel) kernels: same greedy text as the golden generation, and logits no
     further from the scalar reference path than the reference's own AVX2 path is (order band)."""
     from crabml_b200 import CudaTensor
     path = fixture_path(fname)

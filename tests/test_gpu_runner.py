@@ -1,5 +1,5 @@
 """The C++ Llama2Runner replay (crabml_b200/csrc/host/llama2_runner.cpp, the product's host side) end to end:
-golden generations of the reference (llama2.rs:673-703), bit-identical logits in exact_order mode, and a
+golden generations of the GGUF test models, bit-identical logits in exact_order mode, and a
 Llama-2-7B-SHAPED layer on the synthetic weights bench.py uses (BASELINE.json configs 2-4 at full size)."""
 import os
 
@@ -137,7 +137,7 @@ def test_lazy_fused_graph_mode_golden_generation(fixture_path, fname, text, ids,
 
 def test_lazy_mode_matches_eager_ops_through_python_mirror(fixture_path):
     """The recorder is transparent for arbitrary call sequences: the Python replay (not the C++ runner), with debug
-    taps forcing flushes at odd places, gives the reference's golden text."""
+    taps forcing flushes at odd places, gives the golden generation."""
     from crabml_b200 import CudaTensor
     path = fixture_path("tinyllamas-stories-15m-q8_0.gguf")
     gm = GGUFModel(path)
@@ -207,7 +207,7 @@ def test_both_persistent_kernels_bit_identical_on_7b_shapes(tmp_path, wt, ct):
 @pytest.mark.parametrize("fname", ["tinyllamas-stories-15m-q8_0.gguf", "tinyllamas-stories-15m-q4_0.gguf"])
 @pytest.mark.parametrize("f16_kv", [False, True])
 def test_execution_modes_bit_identical_on_fixture(fixture_path, fname, f16_kv):
-    """eager / CUDA-graph / megakernel on the reference's own GGUF fixtures (head_dim 48: unquantised attention output path,
+    """eager / CUDA-graph / megakernel on the GGUF test models (head_dim 48: unquantised attention output path,
     rows of 288 and 768: ragged last group), 24 positions so the softmax spans more than one warp."""
     from crabml_b200 import runner as R
     path = fixture_path(fname)
@@ -255,7 +255,7 @@ def test_device_side_greedy_loop_equals_the_host_sampled_loop(fixture_path, mode
         r2.close()
         assert ids == want_ids
         np.testing.assert_array_equal(logits.view(np.uint32), np.stack(want_logits).view(np.uint32))
-        assert ids[:11] == CASES[0][2]                      # and they are the reference's golden generation
+        assert ids[:11] == CASES[0][2]                      # and they are the golden generation
     finally:
         dev.close()
 

@@ -1,7 +1,7 @@
 """Host logic of the product's C++ Llama2Runner replay (crabml_b200/csrc/host/llama2_runner.cpp) on CPU: built against a mock
 of the C ABI that only records calls, its op trace must equal, call for call (op, shapes, strides, dtypes, scalars, tap names),
-the trace of the Python replay of the reference's forward() (oracle/llama_replay.py -- the replay that reproduces the
-reference's golden generations in tests/test_oracle_golden_text.py) run on a trace-only tensor class.  Covers the
+the trace of the Python replay of the reference's forward() (oracle/llama_replay.py -- the replay that reproduced the
+reference's golden generations on its trained models) run on a trace-only tensor class.  Covers the
 single-device order (llama2.rs:184-281, 527-638) and the sharded insertion points (all_reduce after wo / ffn_down,
 all_gather of the logits)."""
 import ctypes as C

@@ -3,13 +3,14 @@ chaotic w.r.t. f32 summation order.  The truncating Q8_0 activation quantizer (b
 and the f16 exp LUT (cpu_device.rs:108-115) amplify 1e-7 perturbations, so the reference's own scalar
 (buf_q8_0.rs:275-286) and AVX2 (buf_q8_0.rs:228-272) vec_dot orders -- both exercised by its CI
 (.github/workflows/ci.yml:51-57) -- give logits that differ by percents, while the greedy text is equal.
-Hence: fast GPU kernels are held to op-level parity + this band; the 1e-3 bar is proven in exact_order mode."""
+Hence: fast GPU kernels are held to op-level parity + this band; the 1e-3 bar is proven in exact_order mode.
+Measured on the Q8_0 test model of tests/synth_model.py (the reference's trained fixture gave 1.6-4.1 %)."""
 import numpy as np
 
 from oracle import oracle as oc
 from oracle.llama_replay import GGUFModel, Llama2Runner, load_weights
 from oracle.tensor_ref import OracleDevice, OracleTensor
-from tests.test_oracle_golden_text import PROMPT_IDS
+from tests.test_oracle_golden_text import CASES, PROMPT_IDS
 
 
 def order_band(path, n_pos=len(PROMPT_IDS)):
@@ -29,4 +30,4 @@ def test_reference_scalar_vs_avx2_order_band(fixture_path):
     assert band.max() < 0.1
     # ... yet the sampled token (after the last prompt position) agrees, which is all the reference's tests
     # check; at teacher-forced positions even the argmax may flip
-    assert am_a[-1] == am_b[-1] == 29941
+    assert am_a[-1] == am_b[-1] == CASES[0][2][0]
